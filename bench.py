@@ -570,6 +570,19 @@ def streams_leg(torch, dist, ctx, abi, lib, setup, dev, world, rank, total_strea
 
 
 KERNELS = ["k_phaseA_transform", "k_ampmax", "k_phaseA_psy", "k_floor1_fit", "k_floor1_render", "k_cqn"]
+DUMP_BLOCKS = 2048
+
+
+def dump_outputs(torch, path, outs, nb, prefix=""):
+    """Write what a step returned, for comparing two builds output for output: every output array on the same
+    seeded sample of DUMP_BLOCKS blocks (with the same --blocks, the same blocks in every run), as float64 (exact
+    for the int32 and float32 outputs), and the sampled block indices (block_index.npy); about 36 MB for stereo."""
+    os.makedirs(path, exist_ok=True)
+    sel = np.sort(np.random.default_rng(1234).choice(nb, size=min(DUMP_BLOCKS, nb), replace=False))
+    tsel = torch.from_numpy(sel).to(next(iter(outs.values())).device)
+    np.save(os.path.join(path, prefix + "block_index.npy"), sel.astype(np.float64))
+    for name, t in outs.items():
+        np.save(os.path.join(path, prefix + name + ".npy"), t[tsel].cpu().numpy().astype(np.float64))
 
 
 def run_ours(args):
@@ -631,6 +644,9 @@ def run_ours(args):
     barrier()
     ms = e0.elapsed_time(e1)
     launches = ctx.launch_count() - l0
+    if args.dump_outputs:                # the last timed step's outputs, before anything else runs the chain again
+        dump_outputs(torch, args.dump_outputs, {"posts": posts, "nonzero": nonzero, "iwork": iwork, "ampmax_out": amp},
+                     nb, "" if world == 1 else "rank%d_" % rank)
     if rank == 0:
         # the timed region is ~0.1 s: keep the same load running (untimed) until a few clock samples exist
         t_end = time.time() + 2.0
@@ -813,6 +829,8 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the informational configs 2/4")
     ap.add_argument("--streams", type=int, default=10000, help="configs[4]: streams of the fixed mixed-block job (0 = skip)")
     ap.add_argument("--stream-blocks", type=int, default=50, help="long-block lengths per stream of that job")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's outputs "
+                    "(posts, nonzero, iwork, ampmax_out) to DIR/<name>.npy")
     ap.add_argument("--ref-blocks-per-core", type=int, default=2048,
                     help="CPU arms: long stereo blocks per pinned process per step (about 0.4 s of work)")
     if len(sys.argv) > 1 and sys.argv[1] == "--cpu-worker":

@@ -1,13 +1,13 @@
 """Block planning (SURVEY §8 a15): the oracle's restatement of what vorbis_analysis_blockout decides per block
 (W, lW, nW, blocktype, position) must equal the reference's own block sequence, captured while the unmodified
-reference encodes a stream through its public API (oracle/_ref).  Needs /root/reference (oracle/_ref)."""
+reference encodes a stream through its public API.  The reference's sequences are recorded in
+tests/golden/ref_records.xz by tests/golden/make_golden_ref.py (see tests/refrec.py)."""
 import numpy as np
 import pytest
 
+import refrec
 from conftest import probe_signal
-from oracle import pyoracle, pyref
-
-pytestmark = pytest.mark.skipif(not pyref.available(), reason="oracle/_ref not built (no /root/reference)")
+from oracle import pyoracle
 
 GRID = [(2, 44100, .5), (1, 44100, .4), (2, 44100, .1), (1, 22050, .3), (6, 48000, .2), (2, 48000, .9), (2, 32000, 0.)]
 
@@ -25,29 +25,32 @@ def burst_signal(ch, rate, secs, seed):
     return pcm
 
 
-def reference_stream(ch, rate, q, pcm, fields=("pcm",)):
-    r = pyref.Ref(ch, rate, q)
-    cap = r.encode_capture(pcm, fields=fields, timeline=True)
-    return r, cap
+def plan_signal(ch, rate, mode):
+    return probe_signal(ch, rate, 1.5, 7) if mode == "probe" else burst_signal(ch, rate, 1.5, 7)
+
+
+def config1_signal():
+    t = np.arange(44100)
+    return (0.8 * np.sin(2 * np.pi * 440.0 * t / 44100.0)).astype(np.float32)[None]
 
 
 @pytest.mark.parametrize("mode", ["probe", "bursts"])
 @pytest.mark.parametrize("ch,rate,q", GRID)
 def test_oracle_plan_equals_reference_block_sequence(ch, rate, q, mode):
-    pcm = probe_signal(ch, rate, 1.5, 7) if mode == "probe" else burst_signal(ch, rate, 1.5, 7)
-    r, cap = reference_stream(ch, rate, q, pcm)
-    o = pyoracle.Oracle(r.setup())
-    tl = cap["timeline"]
+    rec = refrec.Case("plan", ch, rate, q, mode)
+    setup = refrec.setup(ch, rate, q)
+    tl = refrec.timeline(rec, plan_signal(ch, rate, mode), setup.blocksize(1) // 2)
+    o = pyoracle.Oracle(setup)
     mark, nsteps = o.timeline_marks(tl[None])
-    plan, nb = o.plan_blocks(mark, nsteps, [tl.shape[1]], [cap["eof"]])
-    k = cap["nblocks"]
-    assert nb[0] == k and (cap["W"] == 0).sum() >= 5           # the signals do switch block sizes
+    plan, nb = o.plan_blocks(mark, nsteps, [tl.shape[1]], [int(rec["eof"])])
+    k = int(rec["nblocks"])
+    assert nb[0] == k and (rec["W"] == 0).sum() >= 5           # the signals do switch block sizes
     for name in ("W", "lW", "nW", "blocktype"):
-        assert np.array_equal(plan[0, :k][name], cap[name][:k]), name
+        assert np.array_equal(plan[0, :k][name], rec[name]), name
     for b in range(k):                                          # positions: the block is that slice of the timeline
-        N = r.bs[cap["W"][b]]
+        N = setup.blocksize(int(rec["W"][b]))
         p = plan[0, b]["pos"]
-        assert np.array_equal(cap["pcm"][b][:, :N], tl[:, p:p + N]), "block %d position" % b
+        rec.check(tl[:, p:p + N], "block_%d" % b, "block %d position" % b)
 
 
 def test_config1_plumbing_numbers():
@@ -57,13 +60,13 @@ def test_config1_plumbing_numbers():
     1705 packet bytes.  (SURVEY §8d quotes 47 / 2+45 / 1851 from a survey-time probe whose source was not
     kept; block count and bytes depend on the write chunking - 45..46 blocks, 1615..1705 bytes for chunks
     of 256..44100 samples - so the pinned numbers are the ones this repository can reproduce.)"""
-    t = np.arange(44100)
-    pcm = (0.8 * np.sin(2 * np.pi * 440.0 * t / 44100.0)).astype(np.float32)[None]
-    r, cap = reference_stream(1, 44100, .4, pcm)
-    assert cap["nblocks"] == 46
-    assert int((cap["W"] == 0).sum()) == 2 and int((cap["W"] == 1).sum()) == 44
-    assert cap["bytes"] == 1705
-    o = pyoracle.Oracle(r.setup())
-    mark, nsteps = o.timeline_marks(cap["timeline"][None])
-    plan, nb = o.plan_blocks(mark, nsteps, [cap["timeline"].shape[1]], [cap["eof"]])
-    assert nb[0] == 46 and np.array_equal(plan[0, :46]["W"], cap["W"])
+    rec = refrec.Case("plan", 1, 44100, .4, "config1")
+    assert int(rec["nblocks"]) == 46
+    assert int((rec["W"] == 0).sum()) == 2 and int((rec["W"] == 1).sum()) == 44
+    assert int(rec["bytes"]) == 1705
+    setup = refrec.setup(1, 44100, .4)
+    tl = refrec.timeline(rec, config1_signal(), setup.blocksize(1) // 2)
+    o = pyoracle.Oracle(setup)
+    mark, nsteps = o.timeline_marks(tl[None])
+    plan, nb = o.plan_blocks(mark, nsteps, [tl.shape[1]], [int(rec["eof"])])
+    assert nb[0] == 46 and np.array_equal(plan[0, :46]["W"], rec["W"])
