@@ -12,7 +12,8 @@ from oracle import pyref
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("ch,rate,q", [(2, 44100, 0.5), (1, 44100, 0.4), (2, 44100, 0.1), (6, 48000, 0.2)])
+@pytest.mark.parametrize("ch,rate,q", [(2, 44100, 0.5), (1, 44100, 0.4), (2, 44100, 0.1), (6, 48000, 0.2),
+                                      (2, 44100, -0.1), (2, 96000, 0.7)])
 def test_encoder_packets_identical(cuda_ok, ch, rate, q):
     if not (pyref.available() and pyref.dropin_available()):
         pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
@@ -48,7 +49,8 @@ def _stock_summary(ch, rate, q, pcm):
     return nb, h.value, b.value, c.value
 
 
-@pytest.mark.parametrize("ch,rate,q", [(2, 44100, 0.5), (1, 44100, 0.4), (2, 44100, 0.1), (6, 48000, 0.2)])
+@pytest.mark.parametrize("ch,rate,q", [(2, 44100, 0.5), (1, 44100, 0.4), (2, 44100, 0.1), (6, 48000, 0.2),
+                                      (2, 44100, -0.1), (2, 96000, 0.7)])
 def test_block_seam_packets_identical(cuda_ok, ch, rate, q):
     """SURVEY §8b seam 1: vorbis_analysis through vb200_mapping0_exportbundle.forward - ONE vb200_encode_dsp call per
     block (one H2D, the chain kernels, one D2H), then the reference's own floor1_encode / residue forward for the

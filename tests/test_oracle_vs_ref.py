@@ -12,13 +12,16 @@ from conftest import probe_signal
 from vorbis_b200 import abi, lib as vlib
 
 GRID = [(2, 44100, 0.5), (1, 44100, 0.4), (2, 44100, 0.1), (2, 44100, 0.3), (1, 44100, 0.2),
-        (2, 48000, 0.9), (2, 32000, 0.0), (1, 22050, 0.3)]
+        (2, 48000, 0.9), (2, 32000, 0.0), (1, 22050, 0.3), (2, 44100, -0.1), (1, 44100, -0.1), (4, 44100, 0.5)]
 FLOOR1_ARGS = [(2, 44100, 0.5), (6, 48000, 0.2), (2, 32000, -0.1), (1, 16000, 0.5), (2, 96000, 0.7)]
-ENCODE_ARGS = [(2, 44100, 0.5), (2, 44100, 0.1), (1, 44100, 0.4), (6, 48000, 0.2)]
-MANAGED_ARGS = [(2, 44100, 0.5), (1, 44100, 0.4), (6, 48000, 0.2)]
-ENVELOPE_ARGS = [(2, 44100, 0.5), (1, 44100, 0.4), (6, 48000, 0.2), (1, 22050, 0.3), (2, 32000, 0.0), (2, 96000, 0.7)]
-INVERSE2_ARGS = [(2, 44100, 0.5), (6, 48000, 0.2), (1, 22050, 0.3)]
-RESIDUE_ARGS = [(2, 44100, 0.5), (1, 44100, 0.4), (6, 48000, 0.2), (1, 22050, 0.3), (2, 44100, 0.1)]
+ENCODE_ARGS = [(2, 44100, 0.5), (2, 44100, 0.1), (1, 44100, 0.4), (6, 48000, 0.2), (2, 44100, -0.1), (6, 48000, -0.1),
+               (8, 48000, 0.3)]
+MANAGED_ARGS = [(2, 44100, 0.5), (1, 44100, 0.4), (6, 48000, 0.2), (2, 44100, -0.1)]
+ENVELOPE_ARGS = [(2, 44100, 0.5), (1, 44100, 0.4), (6, 48000, 0.2), (1, 22050, 0.3), (2, 32000, 0.0), (2, 96000, 0.7),
+                 (2, 44100, -0.1)]
+INVERSE2_ARGS = [(2, 44100, 0.5), (6, 48000, 0.2), (1, 22050, 0.3), (2, 44100, -0.1)]
+RESIDUE_ARGS = [(2, 44100, 0.5), (1, 44100, 0.4), (6, 48000, 0.2), (1, 22050, 0.3), (2, 44100, 0.1), (2, 44100, -0.1),
+                (4, 44100, 0.5)]
 ids = lambda g: "ch%d_%d_q%g" % g  # noqa: E731
 
 

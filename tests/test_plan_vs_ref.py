@@ -9,7 +9,8 @@ import refrec
 from conftest import probe_signal
 from oracle import pyoracle
 
-GRID = [(2, 44100, .5), (1, 44100, .4), (2, 44100, .1), (1, 22050, .3), (6, 48000, .2), (2, 48000, .9), (2, 32000, 0.)]
+GRID = [(2, 44100, .5), (1, 44100, .4), (2, 44100, .1), (1, 22050, .3), (6, 48000, .2), (2, 48000, .9), (2, 32000, 0.),
+        (2, 44100, -.1)]
 
 
 def burst_signal(ch, rate, secs, seed):
